@@ -175,6 +175,25 @@ def build_env_maps_gpu(ctx, vq, torch, hdri_w=2048, hdri_h=1024, diff_res=64, sp
     return keep
 
 
+DUMP_PIXELS = 1 << 21       # 2M pixels x float4 = 32 MB (+ 16 MB of indices): within 64 MB for the 4K and the 8K frame alike
+DUMP_SEED = 0
+
+
+def dump_sample_index(torch, frame):
+    """The fixed sample of the frame (H x W x 4) that --dump-outputs writes: DUMP_PIXELS flat pixel indices y * W + x drawn
+    without replacement from a generator seeded with DUMP_SEED, sorted, on the frame's device."""
+    h, w, _ = frame.shape
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, size=min(DUMP_PIXELS, h * w), replace=False))
+    return torch.from_numpy(idx).to(frame.device)
+
+
+def write_dump(out_dir, idx, px):
+    """frame_sample.npy: the RGBA of the sampled pixels (N x 4 float32); frame_sample_index.npy: their flat indices (float64, exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frame_sample.npy"), px.cpu().numpy().astype(np.float32))
+    np.save(os.path.join(out_dir, "frame_sample_index.npy"), idx.cpu().numpy().astype(np.float64))
+
+
 def time_gpu(torch, fn, iters, warmup=3, min_warm_ms=30.0, min_timed_ms=20.0):
     """CUDA-event timing on the current stream. Warm-up runs at least `warmup` launches AND `min_warm_ms` of GPU work (the
     SM clock needs a few ms of load to leave its idle state after host-side input generation); the timed region is at
@@ -785,7 +804,7 @@ def run_reference(args):
     planes, pf, pv, a = _cpu_workload()
     port = text = None
     try:
-        port = _cpu_arm("port", max(2, args.steps // 4), 1, planes, pf, pv, a, budget_s=10.0)
+        port = _cpu_arm("port", args.steps, args.warmup, planes, pf, pv, a, budget_s=10.0)
     except Exception as ex:
         print(f"# multi-process port unavailable ({ex!r})", file=sys.stderr)
     try:
@@ -843,7 +862,11 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "cpu-port"])
     ap.add_argument("--no-extra", action="store_true", help="skip the per-kernel extra section")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed seeded sample of the frame the last "
+                    "step computed to DIR/*.npy (inputs are seeded: two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's frame: it needs --impl ours")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         return run_reference(args)
@@ -912,6 +935,8 @@ def main():
         if dist: dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item()) / n
 
+    # what the caller of the timed step receives: the lit frame (at N > 1 the assembled frame every rank holds)
+    dump_idx = dump_sample_index(torch, out if world == 1 else frame) if args.dump_outputs and rank == 0 else None
     for _ in range(args.warmup):
         step()
     sampler = ClockSampler(local); sampler.start()
@@ -919,12 +944,17 @@ def main():
     lt0 = vq.launch_count()
     ms_step = timed(step, args.steps)
     timed_launches = vq.launch_count() - lt0
+    # gathered on the stream right behind the last timed step, before the clock tail below overwrites `out`
+    dump_px = (out if world == 1 else frame).reshape(-1, 4)[dump_idx] if dump_idx is not None else None
     # keep the GPU busy a little longer so that the clock sampler sees the load even for short runs
     t_end = time.time() + 0.4
     while time.time() < t_end:
         kernel_only()
     torch.cuda.synchronize()
     clocks = sampler.stop()
+    if dump_px is not None:
+        write_dump(args.dump_outputs, dump_idx, dump_px)
+        del dump_px
     px_all = FW * FH
     value = px_all / ms_step / 1e3   # Mpixels/s
     ms_kernel = timed(kernel_only, args.steps) if world > 1 else ms_step

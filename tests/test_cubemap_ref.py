@@ -10,11 +10,13 @@ import numpy as np
 import pytest
 
 import oracle_lib as orc
+import ref_golden as rg
 
 LIB = os.path.join(orc.ORACLE_DIR, "_ref", "libvqcuberef.so")
-pytestmark = pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/libvqcuberef.so not built (needs /root/reference at build time)")
+needs_ref = pytest.mark.skipif(not os.path.exists(LIB), reason="oracle/_ref/libvqcuberef.so not built (needs the engine sources at build time)")
 
 
+@needs_ref
 def test_face_view_matrices_are_the_d3d_cube_convention():
     ref = C.CDLL(LIB)
     want = {0: (1, 0, 0), 1: (-1, 0, 0), 2: (0, 1, 0), 3: (0, -1, 0), 4: (0, 0, 1), 5: (0, 0, -1)}   # RIGHT LEFT UP DOWN FRONT BACK
@@ -26,9 +28,11 @@ def test_face_view_matrices_are_the_d3d_cube_convention():
         assert np.allclose(m[:3, :3] @ m[:3, :3].T, np.eye(3)) and np.array_equal(m[3], np.float32([0, 0, 0, 1]))
 
 
-@pytest.mark.parametrize("res", [1, 2, 8, 64, 512])
+@needs_ref
+@pytest.mark.parametrize("res", rg.CUBE_RES)
 def test_texel_directions_equal_the_reference_matrices(res):
     ref = C.CDLL(LIB)
+    assert rg.reference("cube_dirs", res) == rg.stored("cube_dirs", res)
     o = orc.lib()
     a, b = np.zeros(3, np.float32), np.zeros(3, np.float32)
     pts = sorted({0, res - 1, res // 2, res // 3, (2 * res) // 3})
@@ -43,3 +47,9 @@ def test_texel_directions_equal_the_reference_matrices(res):
                 o.orc_direction_to_cube_face(orc._p(b), C.byref(f), C.byref(sx), C.byref(sy))
                 assert f.value == face
                 assert abs((sx.value * 0.5 + 0.5) * res - (px + 0.5)) < 1e-3 and abs((0.5 - sy.value * 0.5) * res - (py + 0.5)) < 1e-3
+
+
+@pytest.mark.parametrize("res", rg.CUBE_RES)
+def test_texel_directions_equal_the_stored_reference(res):
+    """the oracle's texel directions == the reference's, as stored in tests/golden/ref_golden.json"""
+    assert rg.port("cube_dirs", res) == rg.stored("cube_dirs", res)

@@ -7,6 +7,8 @@ import os
 import numpy as np
 import pytest
 
+import ref_golden as rg
+
 
 @pytest.fixture(scope="module")
 def ref(orc):
@@ -23,7 +25,7 @@ def _img(w, h, seed):
     return a
 
 
-@pytest.mark.parametrize("w,h", [(64, 8), (7, 3), (300, 5), (8, 1), (129, 2)])
+@pytest.mark.parametrize("w,h", rg.IMG_LOAD)
 def test_load_from_file_texels_and_max_luminance(ref, vq, tmp_path, w, h):
     orc = ref
     path = str(tmp_path / f"in_{w}x{h}.hdr")
@@ -34,29 +36,32 @@ def test_load_from_file_texels_and_max_luminance(ref, vq, tmp_path, w, h):
     assert rc == 0 and texels is not None
     assert np.array_equal(texels.view(np.uint32), mine.view(np.uint32))
     assert np.float32(lum) == np.float32(my_lum)           # Image::MaxLuminance == CalculateMaxLuminance restated
+    assert rg.reference("image_load", (w, h)) == rg.stored("image_load", (w, h))
     info, _ = vq.hdr_parse(data)                           # the product's host parser sees the same image
     assert (info.width, info.height) == (w, h)
 
 
-@pytest.mark.parametrize("w,h,ow,oh", [(64, 32, 32, 16), (100, 37, 41, 13), (128, 64, 16, 8), (33, 17, 33, 9)])
+@pytest.mark.parametrize("w,h,ow,oh", rg.IMG_RESIZE)
 def test_create_resized_image(ref, w, h, ow, oh):
     a = _img(w, h, w * 3 + h)
     assert np.array_equal(ref.ref_image_resize(a, ow, oh).view(np.uint32), ref.resize_downsample(a, ow, oh).view(np.uint32))
+    assert rg.reference("image_resize", (w, h, ow, oh)) == rg.stored("image_resize", (w, h, ow, oh))
 
 
-@pytest.mark.parametrize("w,h", [(64, 8), (7, 3), (300, 5)])
+@pytest.mark.parametrize("w,h", rg.IMG_SAVE)
 def test_save_to_disk_is_byte_identical(ref, vq, tmp_path, w, h):
     a = _img(w, h, 11 * w + h)
     path = str(tmp_path / "out.hdr")
     assert ref.ref_image_save(path, a)                     # Image::SaveToDisk
     data = open(path, "rb").read()
-    assert data == ref.hdr_encode(a)
+    assert data == ref.hdr_encode(a) and rg.sha(data) == rg.stored("image_save", (w, h))
     assert data == vq.hdr_pack_file(ref.linear_to_rgbe(a))  # the product's host packer on the oracle's RGBE texels
 
 
 def test_calculate_mip_level_count(ref, vq):
-    for w, h in [(2048, 1024), (4096, 2048), (4096, 4096), (512, 512), (1, 1), (3, 1000), (8192, 4096), (640, 360)]:
+    for w, h in rg.MIP_COUNT:
         want = ref.ref_mip_level_count(w, h)               # Image::CalculateMipLevelCount
+        assert want == rg.stored("mip_count", (w, h))
         assert want == int(ref.lib().orc_mip_level_count(w, h)) == vq.mip_level_count(w, h), (w, h)
 
 
@@ -72,3 +77,17 @@ def test_engine_downsize_flow_4k_to_1k(ref, tmp_path):
     assert ref.ref_image_save(lo, small)
     rc, dec, _ = ref.hdr_decode(open(hi, "rb").read())
     assert open(lo, "rb").read() == ref.hdr_encode(ref.resize_downsample(dec, 128, 64))
+    assert rg.sha(open(lo, "rb").read()) == rg.stored("downsize_flow", (512, 256))
+
+
+@pytest.mark.parametrize("kind,case", [("image_load", c) for c in rg.IMG_LOAD] + [("image_resize", c) for c in rg.IMG_RESIZE]
+                         + [("image_save", c) for c in rg.IMG_SAVE] + [("downsize_flow", (512, 256))])
+def test_image_class_outputs_equal_the_stored_reference(kind, case):
+    """LoadFromFile texels + MaxLuminance, CreateResizedImage, SaveToDisk bytes and the 4k->1k-style downsize flow of the
+    reference's Image class (stored in tests/golden/ref_golden.json) == the oracle's decode / resize / encode"""
+    assert rg.port(kind, case) == rg.stored(kind, case)
+
+
+def test_calculate_mip_level_count_equals_the_stored_reference(orc, vq):
+    for w, h in rg.MIP_COUNT:
+        assert rg.stored("mip_count", (w, h)) == int(orc.lib().orc_mip_level_count(w, h)) == vq.mip_level_count(w, h), (w, h)

@@ -5,6 +5,8 @@ stand-ins) — against the oracle's restatements: the HDRI MIN pyramid (K11) and
 import numpy as np
 import pytest
 
+import ref_golden as rg
+
 
 @pytest.fixture(scope="module")
 def ref(orc):
@@ -13,7 +15,7 @@ def ref(orc):
     return orc
 
 
-@pytest.mark.parametrize("w,h", [(64, 32), (256, 128), (16, 16), (128, 2), (2048, 1024)])
+@pytest.mark.parametrize("w,h", rg.MIP_HDRI)
 def test_hdri_min_pyramid_equals_reference_mip_image(ref, vq, w, h):
     """K11's oracle (MipImage_MinFilter applied down the pyramid, TextureManager.cpp:714-727) == the reference's MipImage
     applied level after level, bit for bit, for as long as both dimensions stay even"""
@@ -31,9 +33,10 @@ def test_hdri_min_pyramid_equals_reference_mip_image(ref, vq, w, h):
         mine = pyr[off: off + lw * lh].reshape(lh, lw, 4)
         assert np.array_equal(mine.view(np.uint32), cur.view(np.uint32)), (l, lw, lh)
     assert l >= 2 or min(w, h) <= 2
+    assert rg.reference("mip_hdri", (w, h)) == rg.stored("mip_hdri", (w, h))
 
 
-@pytest.mark.parametrize("w,h", [(64, 64), (256, 32), (16, 2), (1024, 1024)])
+@pytest.mark.parametrize("w,h", rg.MIP_RGBA8)
 def test_rgba8_box_chain_equals_reference_mip_image(ref, vq, w, h):
     rng = np.random.default_rng(w * 7 + h)
     img = rng.integers(0, 256, (h, w, 4), dtype=np.uint8)
@@ -48,3 +51,10 @@ def test_rgba8_box_chain_equals_reference_mip_image(ref, vq, w, h):
         off = vq.pyramid_offset(w, h, l) * 4
         mine = chain[off: off + lw * lh * 4].reshape(lh, lw, 4)
         assert np.array_equal(mine, cur), (l, lw, lh)
+    assert rg.reference("mip_rgba8", (w, h)) == rg.stored("mip_rgba8", (w, h))
+
+
+@pytest.mark.parametrize("kind,case", [("mip_hdri", c) for c in rg.MIP_HDRI] + [("mip_rgba8", c) for c in rg.MIP_RGBA8])
+def test_mip_chains_equal_the_stored_reference(kind, case):
+    """every even-sized level of the oracle's chains == the reference's MipImage output stored in tests/golden/ref_golden.json"""
+    assert rg.port(kind, case) == rg.stored(kind, case)

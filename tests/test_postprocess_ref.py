@@ -10,6 +10,8 @@ import subprocess
 import numpy as np
 import pytest
 
+import ref_golden as rg
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -20,19 +22,18 @@ def pp(orc):
     return orc.pp_ref()
 
 
-@pytest.mark.parametrize("args", [(1920, 1080, 1920, 1080, 3840, 2160), (1478, 831, 1920, 1080, 1920, 1080), (1280, 720, 1280, 720, 2560, 1440),
-                                  (2227, 1253, 3840, 2160, 3840, 2160), (960, 540, 960, 540, 3840, 2160)])
+@pytest.mark.parametrize("args", rg.EASU)
 def test_easu_constant_block(pp, vq, args):
     con = (C.c_uint * 16)()
     pp.vqpp_easu(con, *[C.c_uint(a) for a in args])
-    assert list(con) == list(vq.fsr_easu_con(*[float(a) for a in args]))
+    assert list(con) == list(vq.fsr_easu_con(*[float(a) for a in args])) == rg.stored("easu", args)
 
 
 @pytest.mark.parametrize("stops", [0.0, 0.2, 0.5, 1.0, 2.0, 0.01])
 def test_rcas_constant_block_and_sharpness_conversion(pp, vq, stops):
     con = (C.c_uint * 4)()
     pp.vqpp_rcas(con, C.c_float(stops))
-    assert list(con) == list(vq.fsr_rcas_con(stops))
+    assert list(con) == list(vq.fsr_rcas_con(stops)) == rg.stored("rcas", stops)
     lin = pp.vqpp_rcas_linear_from_stops(C.c_float(stops))
     assert lin == pytest.approx(0.5 ** stops, rel=1e-6)
     if stops > 0:
@@ -72,3 +73,10 @@ int main() {
     assert lines[1].split() == [f"{w:08x}" for w in rcas]
     assert float(lines[2]) == pytest.approx(pp.vqpp_rcas_linear_from_stops(C.c_float(0.37)), rel=1e-6)
     assert float(lines[3]) == pytest.approx(pp.vqpp_rcas_stops_from_linear(C.c_float(0.3)), rel=1e-5)
+
+
+@pytest.mark.parametrize("kind,case", [("easu", a) for a in rg.EASU] + [("rcas", s) for s in rg.RCAS])
+def test_constant_blocks_equal_the_stored_reference(vq, kind, case):
+    """vq_fsr_easu_con / vq_fsr_rcas_con == the blocks UpdateEASUConstantBlock / UpdateRCASConstantBlock filled (stored in
+    tests/golden/ref_golden.json)"""
+    assert rg.port(kind, case) == rg.stored(kind, case)
