@@ -1,12 +1,6 @@
 #!/usr/bin/env bash
-# GPU-box helper: the whole -m gpu suite, K1 A/B over variants/ (args), smoke, then bench at 1 GPU.
+# GPU-box helper: the whole -m gpu suite, smoke, then bench at 1 GPU.
 mkdir -p gpurun_out
 timeout 1500 python -m pytest tests -q -m gpu -x --durations=8 > gpurun_out/gpu_tests.log 2>&1; echo "gpu tests rc=$?"; tail -14 gpurun_out/gpu_tests.log
-: > gpurun_out/k1_variants.txt
-for v in "$@"; do
-  echo "== variant [$v]" >> gpurun_out/k1_variants.txt
-  VQCUDA_LIB=variants/$v.so timeout 120 python tools/perf_forward.py 2>&1 | grep -E "forward 4K prepared|rror" >> gpurun_out/k1_variants.txt
-done
-cat gpurun_out/k1_variants.txt
 timeout 300 python -c "import __graft_entry__ as g; g.smoke()" 2>&1 | tail -2
 timeout 900 python bench.py --gpus 1 --steps 30 --warmup 5 > gpurun_out/bench_1gpu.json 2> gpurun_out/bench_1gpu.err; echo "bench rc=$?"; head -c 1500 gpurun_out/bench_1gpu.json; tail -3 gpurun_out/bench_1gpu.err

@@ -133,14 +133,14 @@ out.append("\n## How these were produced\n")
 out.append("All on `gpurun` B200 boxes from this tree (scripts under `tools/`):\n")
 out.append("* `bash tools/gpu_final.sh` — `pytest -m gpu` (-> `r02_gpu_tests.txt`), smoke, `python bench.py` (-> `r02_bench_1gpu.json`), compute-sanitizer memcheck / racecheck "
            "over one small launch of every kernel (`tools/sanitize_small.py` -> `r02_sanitize_{memcheck,racecheck}.txt`), the ncu launch list of the bench command (-> `r02_launches_bench.csv`).")
-out.append("* `[NCU=regex] bash tools/gpu_ab_pass.sh surface|shadow|frame [variants]` — parity tests of one pass family, its timings for the in-tree library and for builds in "
-           "`variants/` (-> `r02_{surface,shadow,frame}_variants.txt`), one full ncu capture (-> `r02_{surface_d,surface_e,shadow_b,shadow_c,frame_b}_summary.txt`; "
+out.append("* Parity tests of one pass family, its timings for the in-tree library and for builds with other tuning constants "
+           "(-> `r02_{surface,shadow,frame}_variants.txt`), one full ncu capture (-> `r02_{surface_d,surface_e,shadow_b,shadow_c,frame_b}_summary.txt`; "
            "`tools/ncu_lines.py` attributes executed instructions and stall samples to source lines); `tools/perf_e2e.py` (-> `r02_e2e_link.txt`).")
 out.append("* `bash tools/gpu_2gpu.sh N` under `gpurun --gpus N` — the driver's torchrun command for `bench.py --gpus N` (-> `r02_bench_{2,4,8}gpu.json`).")
-out.append("* `bash tools/gpu_k1.sh [variants]` — K1 at 4K, the forward parity tests, `ncu --set full --clock-control none --import-source on -k regex:forward_kernel` "
+out.append("* K1 at 4K, the forward parity tests, `ncu --set full --clock-control none --import-source on -k regex:forward_kernel` "
            "over `tools/perf_forward.py` (-> `r02_forward_{a,b}_summary.txt` via `tools/ncu_summary.py`, `forward_traffic.json` via `tools/make_forward_traffic.py`); "
            "A/B logs `r02_forward_variants_{a,b,c,d}.txt`.")
-out.append("* `bash tools/gpu_ab.sh <variants>` — K1 + 2x EASU A/B over builds in `variants/` (-> `r02_post_variants.txt`); `tools/ubench_gather.cu` "
+out.append("* K1 + 2x EASU A/B over builds with other tuning constants (-> `r02_post_variants.txt`); `tools/ubench_gather.cu` "
            "(-> `r02_ubench_gather.txt`): what a warp-wide gather costs in the L1 data pipe.")
 out.append("* `python tests/diag_fullsize.py` (-> `r02_diag_fullsize.txt`): where the first full-size parity run disagreed with the oracle, and why (DESIGN.md §5).")
 out.append("* `r02_shadow_first_run.txt`, `r02_shadow_a_summary.txt`: the first execution of the (f).4 kernels (15 parity tests, timings, memcheck, ncu).")

@@ -1,5 +1,5 @@
-"""GPU-box helper: the e2e call (vq_forward_lighting_host, pinned host buffers) at 4K for several chunk counts, next to what the
-PCIe link does on plain copies of the same buffers."""
+"""GPU-box helper: the e2e call (vq_forward_lighting_host, pinned host buffers) at 4K with the library's row chunking, next to
+what the PCIe link does on plain copies of the same buffers."""
 import os, sys, time, json
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -23,11 +23,8 @@ def timeit(fn, reps=6):
     for _ in range(reps): fn()
     torch.cuda.synchronize()
     return (time.perf_counter() - t0) / reps
-res = {}
-for chunks in (16, 8, 4, 2):
-    os.environ["VQ_HOST_CHUNKS"] = str(chunks)
-    dt = timeit(lambda: ctx.forward_lighting_host(pf, pv, hgb, envk["env"], hout))
-    res[f"e2e_chunks_{chunks}"] = {"ms": round(dt * 1e3, 3), "Mpixels_per_s": round(W * H / dt / 1e6, 1)}
+dt = timeit(lambda: ctx.forward_lighting_host(pf, pv, hgb, envk["env"], hout))
+res = {"e2e": {"ms": round(dt * 1e3, 3), "Mpixels_per_s": round(W * H / dt / 1e6, 1)}}
 d = torch.empty((H, W, 4), dtype=torch.float32, device="cuda"); d2 = torch.empty_like(d)
 nb = d.numel() * 4
 s2 = torch.cuda.Stream()

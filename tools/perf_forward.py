@@ -1,5 +1,5 @@
-"""GPU-box helper: time K1 at 4K (prepared environment), print us + GB/s. Parity of a variant build is checked by the tests:
-   VQCUDA_LIB=variants/<name>.so python -m pytest tests/test_forward_gpu.py -q -m gpu -k "full_size or config3" """
+"""GPU-box helper: time K1 at 4K (prepared environment), print us + GB/s. Parity is checked by the tests:
+   python -m pytest tests/test_forward_gpu.py -q -m gpu -k "full_size or config3" """
 import os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))

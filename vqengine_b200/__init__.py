@@ -15,7 +15,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("VQCUDA_LIB") or os.path.join(_HERE, "libvqcuda.so")   # override only for A/B kernel experiments
+LIB_PATH = os.path.join(_HERE, "libvqcuda.so")
 
 from .shader_data import *          # noqa: F401,F403  (struct mirror + constants: plain data, no library)
 from .shader_data import f32, i32, u32

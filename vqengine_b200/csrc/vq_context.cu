@@ -69,19 +69,6 @@ int vq_ctx_create(int device, VqContext** out_ctx) {
     c->l2_bytes = prop.l2CacheSize;
     if (cudaMalloc(&c->spd_counter, 2 * VQ_SPD_SLOTS * sizeof(uint32_t)) != cudaSuccess) { delete c; vq_set_error("cudaMalloc failed"); return VQ_ERR_OUT_OF_MEMORY; }
     cudaMemset(c->spd_counter, 0, 2 * VQ_SPD_SLOTS * sizeof(uint32_t));
-    {   // persisting-L2 carve-out for K1's sampling copies (vq_forward.cu), OPT-IN (VQ_L2_PERSIST=1): measured on B200 it makes the
-        // 4K pass 27 % SLOWER (331 vs 261 us, profiles/r02_forward_variants_c.txt) — the set-aside takes L2 away from the 531 MB
-        // that stream through per frame, and 102 MB of copies do not fit it anyway. The device limit is process-wide state.
-        const char* e = getenv("VQ_L2_PERSIST");
-        int maxPersist = 0, maxWindow = 0;
-        cudaDeviceGetAttribute(&maxPersist, cudaDevAttrMaxPersistingL2CacheSize, device);
-        cudaDeviceGetAttribute(&maxWindow, cudaDevAttrMaxAccessPolicyWindowSize, device);
-        if (e && e[0] == '1' && maxPersist > 0 && maxWindow > 0 &&
-            cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, (size_t)maxPersist) == cudaSuccess) {
-            c->l2_persist_bytes = (size_t)maxPersist; c->l2_window_max = maxWindow;
-        }
-        cudaGetLastError();
-    }
     c->spd_next = new std::atomic<uint32_t>(0u);
     c->mu = new std::recursive_mutex();
     *out_ctx = c;

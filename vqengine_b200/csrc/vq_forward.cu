@@ -19,10 +19,6 @@
 
 using namespace vq;
 
-#ifndef FWD_BACKOFF
-#define FWD_BACKOFF 128        // ns the producer thread sleeps between polls of an empty[] barrier (0: spin)
-#endif
-
 namespace {
 
 
@@ -208,10 +204,7 @@ struct Acc2 { f2 ax, ay, az, bx, by, bz, cx, cy, cz; };   // sum over lights of 
 // N.H with the oracle's exact operation sequence (correctly rounded div/sqrt, no FMA contraction): V, Wo,
 // N, Wi, H as BRDF.hlsl:166-169 / Lighting.hlsl:312 write them. T_EXACT = 0.02 bounds the fast path's
 // relative error in D by 2*dt/t <= 2*5e-7/0.02 = 5e-5; the slow path runs for < 1 % of pixel-light pairs.
-#ifndef FWD_T_EXACT
-#define FWD_T_EXACT 0.02f
-#endif
-constexpr float T_EXACT = FWD_T_EXACT;
+constexpr float T_EXACT = 0.02f;
 
 // dot_u, sqrt_rn_inrange, rcp_rn_prepare / div_rn_inrange, len2_inrange: vq_common.cuh (shared with the PCF kernel)
 // v / sqrt(dot(v,v)) with correctly rounded sqrt and divisions (== the oracle's normalize)
@@ -347,11 +340,8 @@ __device__ __forceinline__ void shade_all_lights(const Px2& s, Acc2& acc, const 
     const int numPoint = P.numPoint, numSpot = P.numSpot;
     // ---- point lights, then point casters (Lighting.hlsl:308-322; PSMain :310-313,321-340):
     //      in range <=> d2 < d2Limit (== length(Lw-P) < l.range, exactly) ----
-#ifndef FWD_LIGHT_UNROLL
-#define FWD_LIGHT_UNROLL 1      // 2: two lights interleaved (more ILP for the dependent MUFU/FMA chains, ~20 more registers)
-#endif
-    constexpr int kLightUnroll = FWD_LIGHT_UNROLL;
-#pragma unroll kLightUnroll
+    // one light at a time: interleaving two buys ILP for the dependent MUFU/FMA chains at ~20 more registers
+#pragma unroll 1
     for (int i = 0; i < numPoint; ++i) {
         const SPoint l = P.pts[i];                                       // constant bank, warp-uniform index
         const LightVec2 L = light_vector2(s, l.pos);
@@ -417,9 +407,7 @@ __device__ __forceinline__ void mbar_wait_backoff(uint32_t bar, uint32_t parity)
         asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
                      : "=r"(done) : "r"(bar), "r"(parity) : "memory");
         if (done) break;
-#if FWD_BACKOFF
-        __nanosleep(FWD_BACKOFF);
-#endif
+        __nanosleep(128);
     }
 }
 __device__ __forceinline__ uint64_t l2_evict_first_policy() {
@@ -450,15 +438,9 @@ __device__ __forceinline__ void st_stream_hint(float4* p, float4 v, uint64_t pol
 // ITS texels back with LDS when it needs them and releases the stage (empty[] mbarriers) when its pixels are
 // stored. Nothing of the G-buffer is live in registers across the light loop: albedo/metalness/ao, the raw
 // normal and the emissive texel are (re-)read from the stage after it.
-#ifndef FWD_STAGES
-#define FWD_STAGES 2           // shared-memory stages
-#endif
-#ifndef FWD_AHEAD
-#define FWD_AHEAD 1            // tiles requested ahead of the one being shaded (< FWD_STAGES)
-#endif
-#ifndef FWD_CTAS_PER_SM
-#define FWD_CTAS_PER_SM 4
-#endif
+constexpr int FWD_STAGES = 2;          // shared-memory stages
+constexpr int FWD_AHEAD = 1;           // tiles requested ahead of the one being shaded (< FWD_STAGES)
+constexpr int FWD_CTAS_PER_SM = 4;
 static_assert(FWD_AHEAD >= 1 && FWD_AHEAD < FWD_STAGES, "the lookahead must leave at least one stage for the tile being shaded");
 
 // ---- environment taps -----------------------------------------------------------------------------------
@@ -467,24 +449,12 @@ static_assert(FWD_AHEAD >= 1 && FWD_AHEAD < FWD_STAGES, "the lookahead must leav
 struct FaceRec { uint32_t base; uint32_t P; float halfN; float c0; };     // first record of the face, row stride, N/2, N/2 - 0.5
 static_assert(sizeof(FaceRec) == 16, "one LDS.128");
 
-// L1 policy of a gather (A/B on B200, profiles/r02_forward_variants.txt): 0 = allocate, 1 = L1::no_allocate, 2 = L1::evict_last
-#ifndef FWD_L1_DIFF
-#define FWD_L1_DIFF 0
-#endif
-#ifndef FWD_L1_SPEC
-#define FWD_L1_SPEC 1
-#endif
-#ifndef FWD_L1_LUT
-#define FWD_L1_LUT 1
-#endif
-template <int POLICY>
+// L1 policy of a gather (A/B on B200): the diffuse cube's gathers allocate in L1, the specular cube's and the LUT's do not
+template <bool NO_ALLOCATE>
 __device__ __forceinline__ F8 ldg256(const float4* p) {             // 32-byte aligned, read-only path (LDG.E.256)
     F8 r;
-    if (POLICY == 1)
+    if (NO_ALLOCATE)
         asm("ld.global.nc.L1::no_allocate.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-            : "=f"(r.a.x), "=f"(r.a.y), "=f"(r.a.z), "=f"(r.a.w), "=f"(r.b.x), "=f"(r.b.y), "=f"(r.b.z), "=f"(r.b.w) : "l"(p));
-    else if (POLICY == 2)
-        asm("ld.global.nc.L1::evict_last.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
             : "=f"(r.a.x), "=f"(r.a.y), "=f"(r.a.z), "=f"(r.a.w), "=f"(r.b.x), "=f"(r.b.y), "=f"(r.b.z), "=f"(r.b.w) : "l"(p));
     else
         asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
@@ -500,7 +470,7 @@ struct CubeLoad { F8 r0, r1; float fx, fy; };                     // rows j0 and
 // A gather is split into "issue" (address + the 256-bit loads) and "finish" (the lerps) so that the loads of several
 // gathers are in flight before the first one is consumed.
 // maxRec: last record a footprint may start at (clamps the address for NaN/inf directions: no surface => no normal)
-template <int POLICY>
+template <bool NO_ALLOCATE>
 __device__ __forceinline__ CubeLoad cube_issue(const float4* __restrict__ recs, FaceRec f, uint32_t maxRec, float sx, float sy) {
     const float x = fmaf(sx, f.halfN, f.c0), y = fmaf(-sy, f.halfN, f.c0);       // texel space: (s*0.5+0.5)*N - 0.5
     const float xf = floorf(x), yf = floorf(y);                                  // in [-1, N-1] for every finite direction
@@ -508,7 +478,7 @@ __device__ __forceinline__ CubeLoad cube_issue(const float4* __restrict__ recs, 
     L.fx = x - xf; L.fy = y - yf;
     const uint32_t off = min(f.base + (uint32_t)((int)yf + 1) * f.P + (uint32_t)((int)xf + 1), maxRec);
     const float4* p = recs + 2u * off;
-    L.r0 = ldg256<POLICY>(p); L.r1 = ldg256<POLICY>(p + 2u * f.P);
+    L.r0 = ldg256<NO_ALLOCATE>(p); L.r1 = ldg256<NO_ALLOCATE>(p + 2u * f.P);
     return L;
 }
 // bilinear blend of the footprint as packed pairs {x,y}, {z,w} of one pixel: 12 packed operations instead of 18 scalar ones
@@ -528,7 +498,7 @@ __device__ __forceinline__ LutLoad lut_issue(const LutV& l, float u, float v) { 
     LutLoad L;
     L.fx = x - x0; L.fy = y - y0;
     const int cx = min(max((int)x0 + 1, 0), l.w), cy = min(max((int)y0 + 1, 0), l.h);
-    L.q = ldg256<FWD_L1_LUT>(l.q + 2u * (uint32_t)(cy * (l.w + 1) + cx));
+    L.q = ldg256<true>(l.q + 2u * (uint32_t)(cy * (l.w + 1) + cx));
     return L;
 }
 __device__ __forceinline__ float2 lut_finish(const LutLoad& L) {    // record = {p00, p10 | p01, p11} as float2 each
@@ -544,13 +514,9 @@ __device__ __forceinline__ float2 lut_finish(const LutLoad& L) {    // record = 
 //   Ns : the surface normal as normalize(Ns)*|Ns| (within an ulp of the raw texel; it only steers the two cube lookups)
 // The environment lookups of one pixel, split into "issue" (the five 256-bit gathers: diffuse cube x2, specular cube x2, LUT, with
 // their bilinear weights) and "compose" (the blends + the final composition), so that the kernel can put BOTH pixels' gathers in
-// flight before it consumes either (FWD_JOINT_ISSUE): a thread then waits for the L2/HBM latency once per pair instead of once per
+// flight before it consumes either: a thread then waits for the L2/HBM latency once per pair instead of once per
 // pixel (ncu: a third of all stall samples sit on the first use of pixel A's taps and again on pixel B's). Ten 256-bit loads in
 // flight need ~160 registers, i.e. three CTAs per SM instead of four: A/B in profiles/r02_forward_variants_e.txt.
-//   Ns : the surface normal as normalize(Ns)*|Ns| (within an ulp of the raw texel; it only steers the two cube lookups)
-#ifndef FWD_JOINT_ISSUE
-#define FWD_JOINT_ISSUE 1
-#endif
 struct EnvLoads { CubeLoad D, S; LutLoad L; };
 template <bool ROT, bool SPEC>
 __device__ __forceinline__ void env_issue(EnvLoads& E, const FwdParams& P, const FaceRec* __restrict__ sFace, float3 V, float nsnv, float3 Ns, float roughness) {
@@ -558,13 +524,13 @@ __device__ __forceinline__ void env_issue(EnvLoads& E, const FwdParams& P, const
     int face; float sx, sy;
     dir_to_face(Nr, face, sx, sy);
     FaceRec fd; fd.P = (uint32_t)P.diff.res + 2u; fd.base = (uint32_t)face * fd.P * fd.P; fd.halfN = P.diffHalfN; fd.c0 = P.diffHalfN - 0.5f;
-    E.D = cube_issue<FWD_L1_DIFF>(P.diff.p, fd, P.diffMaxRec, sx, sy);
+    E.D = cube_issue<false>(P.diff.p, fd, P.diffMaxRec, sx, sy);
     if (SPEC) {
         const float3 R0 = reflect(-V, Ns);
         const float3 R = ROT ? f3(R0.x * P.cosB - R0.z * P.sinB, R0.y, R0.x * P.sinB + R0.z * P.cosB) : R0;
         dir_to_face(R, face, sx, sy);
         const int mip = min(max((int)(roughness * (float)P.maxLod), 0), P.spec.mips - 1);
-        E.S = cube_issue<FWD_L1_SPEC>(P.spec.p, sFace[face * 16 + mip], P.specMaxRec, sx, sy);
+        E.S = cube_issue<true>(P.spec.p, sFace[face * 16 + mip], P.specMaxRec, sx, sy);
         E.L = lut_issue(P.lut, nsnv, roughness);                                 // (saturate(dot(s.N, V)), roughness)
     }
 }
@@ -620,18 +586,13 @@ __device__ __forceinline__ void finish_pair(const FwdParams& P, const FaceRec* _
     const f2 Nrx = s.Nx * s.nsLen, Nry = s.Ny * s.nsLen, Nrz = s.Nz * s.nsLen;
     EnvLoads eA, eB;
     env_issue<ROT, SPEC>(eA, P, sFace, f3(s.Vx.v.x, s.Vy.v.x, s.Vz.v.x), nsnv.v.x, f3(Nrx.v.x, Nry.v.x, Nrz.v.x), roughness.v.x);
-#if FWD_JOINT_ISSUE
     env_issue<ROT, SPEC>(eB, P, sFace, f3(s.Vx.v.y, s.Vy.v.y, s.Vz.v.y), nsnv.v.y, f3(Nrx.v.y, Nry.v.y, Nrz.v.y), roughness.v.y);
-#endif
     const float4 oA = compose_pixel<SPEC>(P, s.texA, nsnv.v.x, roughness.v.x, ao.v.x, f3(acc.ax.v.x, acc.ay.v.x, acc.az.v.x),
                                           f3(acc.bx.v.x, acc.by.v.x, acc.bz.v.x), f3(acc.cx.v.x, acc.cy.v.x, acc.cz.v.x), eA);
     if (validA) {   // one STG.128 per destination; peer destinations are mapped NVLink addresses (fused compute + gather)
         if (MULTI) { for (int q = 0; q < P.nOut; ++q) st_stream(P.outs[q].row(P.dstRowOffset + y) + xA, oA); }
         else st_stream_hint(P.outs[0].row(P.dstRowOffset + y) + xA, oA, l2_evict_first_policy());
     }
-#if !FWD_JOINT_ISSUE
-    env_issue<ROT, SPEC>(eB, P, sFace, f3(s.Vx.v.y, s.Vy.v.y, s.Vz.v.y), nsnv.v.y, f3(Nrx.v.y, Nry.v.y, Nrz.v.y), roughness.v.y);
-#endif
     const float4 oB = compose_pixel<SPEC>(P, s.texB, nsnv.v.y, roughness.v.y, ao.v.y, f3(acc.ax.v.y, acc.ay.v.y, acc.az.v.y),
                                           f3(acc.bx.v.y, acc.by.v.y, acc.bz.v.y), f3(acc.cx.v.y, acc.cy.v.y, acc.cz.v.y), eB);
     if (validB) {
@@ -989,37 +950,11 @@ int vq_forward_launch_multi(VqContext* ctx, const VqPerFrameData* pf, const VqPe
         VQ_CUDA_OK(cudaFuncSetAttribute(forward_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
         attrSet.store(true, std::memory_order_release);
     }
-    // Experiment kept behind VQ_L2_PERSIST=1 (off by default: it measured 27 % slower, see vq_context.cu): a PERSISTING access-policy
-    // window over the one allocation that holds the sampling copies, as a per-launch attribute (the caller's stream state is not
-    // touched). Without it the G-buffer streams through with evict_first and the copies keep about half their lines in L2
-    // (ncu r02: L2 hit rate 48 %, 135 MB of extra DRAM reads per 4K frame — latency, not bandwidth, at 27 % DRAM utilisation).
-    cudaLaunchAttribute attr[1];
-    unsigned nAttr = 0;
-    if (prepared && ctx->l2_persist_bytes > 0 && ctx->env_used_bytes > 0) {
-        cudaAccessPolicyWindow w;
-        w.base_ptr = ctx->env_all;
-        w.num_bytes = ctx->env_used_bytes < (size_t)ctx->l2_window_max ? ctx->env_used_bytes : (size_t)ctx->l2_window_max;
-        const double ratio = (double)ctx->l2_persist_bytes / (double)w.num_bytes;
-        w.hitRatio = ratio >= 1.0 ? 1.0f : (float)ratio;
-        w.hitProp = cudaAccessPropertyPersisting;
-        w.missProp = cudaAccessPropertyStreaming;
-        attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
-        attr[0].val.accessPolicyWindow = w;
-        nAttr = 1;
-    }
-    auto launch = [&](auto kernel) -> int {
-        cudaLaunchConfig_t cfg;
-        memset(&cfg, 0, sizeof(cfg));
-        cfg.gridDim = dim3(gx, gy); cfg.blockDim = dim3(FWD_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-        cfg.attrs = attr; cfg.numAttrs = nAttr;
-        VQ_CUDA_OK(cudaLaunchKernelEx(&cfg, kernel, P));
-        return VQ_OK;
-    };
+    auto launch = [&](auto kernel) { kernel<<<dim3(gx, gy), FWD_THREADS, smem, stream>>>(P); };
     VQ_REQUIRE(smem <= 96 * 1024, "stage layout exceeds the shared-memory budget");
-    if (shadowed) rc = rot ? launch(forward_kernel<false, true, true>) : launch(forward_kernel<false, false, true>);
-    else if (n_outs > 1) rc = rot ? launch(forward_kernel<true, true>) : launch(forward_kernel<true, false>);
-    else rc = rot ? launch(forward_kernel<false, true>) : launch(forward_kernel<false, false>);
-    if (rc) return rc;
+    if (shadowed) rot ? launch(forward_kernel<false, true, true>) : launch(forward_kernel<false, false, true>);
+    else if (n_outs > 1) rot ? launch(forward_kernel<true, true>) : launch(forward_kernel<true, false>);
+    else rot ? launch(forward_kernel<false, true>) : launch(forward_kernel<false, false>);
     return vq_check_launch("forward_lighting");
 }
 
@@ -1069,14 +1004,13 @@ extern "C" int vq_environment_prepare(VqContext* ctx, const VqEnvironmentMaps* e
     const bool hasSpec = env->irradiance_specular.ptr != nullptr, hasLut = env->brdf_lut.ptr != nullptr;
     if (hasSpec) VQ_REQUIRE(cube_desc_ok(env->irradiance_specular), "bad cubemap descriptor (irradiance_specular)");
     if (hasLut) VQ_REQUIRE(vq_image_ok(env->brdf_lut, 8) && env->brdf_lut.width <= 8192 && env->brdf_lut.height <= 8192, "bad BRDF LUT descriptor");
-    // ONE allocation for the three sampling copies (diffuse | specular | LUT footprints, 256-byte aligned parts): the forward
-    // kernel can then put a single L2 access-policy window over all of its L2-resident side data
+    // ONE allocation for the three sampling copies (diffuse | specular | LUT footprints, 256-byte aligned parts): one buffer
+    // to grow and free instead of three, regrown only when the three together outgrow it
     auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t bD = up(padded_bytes(env->irradiance_diffuse.res, env->irradiance_diffuse.mips));
     const size_t bS = hasSpec ? up(padded_bytes(env->irradiance_specular.res, env->irradiance_specular.mips)) : 0;
     const size_t bL = hasLut ? up(lut_footprint_bytes(env->brdf_lut)) : 0;
     rc = ensure_bytes(&ctx->env_all, &ctx->env_all_bytes, bD + bS + bL); if (rc) return rc;
-    ctx->env_used_bytes = bD + bS + bL;
     ctx->env_diff = ctx->env_all;
     ctx->env_spec = hasSpec ? (char*)ctx->env_all + bD : nullptr;
     ctx->env_lut = hasLut ? (char*)ctx->env_all + bD + bS : nullptr;

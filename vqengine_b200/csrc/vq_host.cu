@@ -3,11 +3,6 @@
 // (upload | shade | download) so that PCIe traffic in both directions overlaps the kernel; with pinned
 // host memory (cudaHostRegister / cudaMallocHost) the copies are truly asynchronous.
 #include "vq_common.cuh"
-#include <stdlib.h>
-
-namespace {
-constexpr int kMaxChunks = 16;
-}
 
 extern "C" int vq_forward_lighting_host(VqContext* ctx, const VqPerFrameData* pf, const VqPerViewLightingData* pv,
                                         const VqGBuffer* hgb, const VqEnvironmentMaps* denv, VqImage hout) {
@@ -47,8 +42,7 @@ extern "C" int vq_forward_lighting_host(VqContext* ctx, const VqPerFrameData* pf
 
     // 8 chunks measured best at 4K (8.16 ms; 16: 8.32, 4: 8.24, 2: 8.71; the link alone moves the 398 MB in 7.19 ms and loses 12 %
     // per direction while both directions are busy: profiles/r02_e2e_link.txt)
-    int chunks = H >= 256 ? 8 : (H >= 16 ? 4 : 1);
-    if (const char* e = getenv("VQ_HOST_CHUNKS")) { const int c = atoi(e); if (c >= 1 && c <= kMaxChunks && c <= H) chunks = c; }   // tuning knob
+    const int chunks = H >= 256 ? 8 : (H >= 16 ? 4 : 1);
     const int rowsPer = (H + chunks - 1) / chunks;
     cudaStream_t sUp = ctx->streams[0], sRun = ctx->streams[1], sDown = ctx->streams[2];
     const VqImage* hp[4] = {&hgb->position_ao, &hgb->normal_roughness, &hgb->albedo_metalness, &hgb->emissive};

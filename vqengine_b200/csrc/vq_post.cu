@@ -112,10 +112,7 @@ __constant__ float c_gauss[11] = {0.224716f, 0.191756f, 0.119146f, 0.053897f, 0.
 // loads are issued into registers before the current row is filtered (software pipelining), results leave through a
 // shared-memory transpose so that the stores are coalesced.
 constexpr int BX_T = 128;            // threads per CTA (4 autonomous warps)
-#ifndef BX_XR_D
-#define BX_XR_D 4
-#endif
-constexpr int BX_XR = BX_XR_D;       // consecutive rows per CTA (software-pipelined)
+constexpr int BX_XR = 4;             // consecutive rows per CTA (software-pipelined)
 constexpr int BX_WW = 128;           // output pixels per warp per row (4 per lane)
 constexpr int BX_W = BX_WW * (BX_T / 32);   // per CTA
 constexpr int BX_SM = BX_WW + 24;    // staged per warp: [-12, BX_WW+12)
@@ -190,14 +187,8 @@ __global__ void __launch_bounds__(BX_T) blur_x_kernel(ImgV in, ImgV out, int siz
 constexpr int BYM_T = 128;          // threads per CTA = columns per CTA
 // A/B on B200 at 4K (us): rows/prefetch 21/21: 47.9 | 42/21: 49.2 | 63/21: 51.0 | 63/7: 57.2 | 126/7: 65.3 | 252/7: 62.5
 // (the shared-memory tile version it replaces: 67.5)
-#ifndef BYM_ROWS_D
-#define BYM_ROWS_D 21
-#endif
-#ifndef BYM_PRE_D
-#define BYM_PRE_D 21
-#endif
-constexpr int BYM_ROWS = BYM_ROWS_D; // output rows per thread (multiple of 21)
-constexpr int BYM_PRE = BYM_PRE_D;   // rows requested ahead of use (divides 21): memory-level parallelism per thread
+constexpr int BYM_ROWS = 21;        // output rows per thread (multiple of 21)
+constexpr int BYM_PRE = 21;         // rows requested ahead of use (divides 21): memory-level parallelism per thread
 
 __global__ void __launch_bounds__(BYM_T) blur_y_kernel(ImgV in, ImgV out, int sizeX, int sizeY) {
     const int x = blockIdx.x * BYM_T + threadIdx.x;
@@ -487,10 +478,7 @@ __global__ void __launch_bounds__(ST_BX * ST_BY) easu_kernel(ImgV in, ImgV out, 
 //   phase 2: one thread per output pixel blends the four analyses with its bilinear weights and runs the 12 taps with
 //            incrementally updated rotated offsets (v(i,j) = v(0,0) + i*A + j*B instead of two dot products per tap).
 // ncu r01: the per-output kernel executed 505 instructions per output pixel; this organisation needs ~60 % of that.
-#ifndef EU_BY_D
-#define EU_BY_D 8
-#endif
-constexpr int EU_BX = 32, EU_BY = EU_BY_D;
+constexpr int EU_BX = 32, EU_BY = 8;
 constexpr int EU_TW = EU_BX + 4, EU_TH = EU_BY + 4;
 
 struct EasuSet { float dirX, dirY, lenX, lenY; };
@@ -526,7 +514,7 @@ __device__ __forceinline__ void easu_tap_v(float3& aC, float& aW, float vx, floa
 }
 
 template <int ADDR>
-__global__ void __launch_bounds__(EU_BX * EU_BY, EU_BY <= 8 ? 4 : 2) easu_up_kernel(ImgV in, ImgV out, EasuCon con) {
+__global__ void __launch_bounds__(EU_BX * EU_BY, 4) easu_up_kernel(ImgV in, ImgV out, EasuCon con) {
     __shared__ float4 tile[EU_TH][EU_TW];          // rgb + luma
     __shared__ float4 sets[4][EU_BY][EU_BX];       // S,T,U,V analyses of candidate texel (fy-fyFirst, fx-fxFirst); SoA: conflict-free
     const int ox0 = blockIdx.x * EU_BX, oy0 = blockIdx.y * EU_BY;
@@ -631,13 +619,8 @@ __global__ void __launch_bounds__(EU_BX * EU_BY, EU_BY <= 8 ? 4 : 2) easu_up_ker
 // {left pixel, right pixel} (FFMA2/FMUL2/FADD2: one issue slot for two pixels). ncu r01: the one-pixel-per-thread kernel issued
 // 485 instructions per output pixel at 77 % issue utilisation (0.62 ms 4K->8K); this one issues ~150.
 // Texels k = -1 and k = W-1 (m likewise) own quads that hang over the image edge: those stores are predicated off.
-#ifndef E2_BY_D
-#define E2_BY_D 4
-#endif
-#ifndef E2_MINB
-#define E2_MINB 8
-#endif
-constexpr int E2_BX = 32, E2_BY = E2_BY_D;             // input texels ('f' candidates) per CTA -> 64 x 2*E2_BY output pixels
+constexpr int E2_BX = 32, E2_BY = 4;                   // input texels ('f' candidates) per CTA -> 64 x 2*E2_BY output pixels
+constexpr int E2_MINB = 8;
 constexpr int E2_TW = E2_BX + 3, E2_TH = E2_BY + 3;    // staged footprint: columns k-1 .. k+2, rows m-1 .. m+2
 
 struct EasuPx2 { f2 dirx, diry, lenx, leny, lob, clp; };
@@ -708,11 +691,8 @@ __global__ void __launch_bounds__(E2_BX * E2_BY, E2_MINB) easu_2x_kernel(ImgV in
         min4 = fmin3(fmin3(xyz(tf), fmin3(xyz(tg), xyz(tj))), xyz(tk));
         max4 = fmax3(fmax3(xyz(tf), fmax3(xyz(tg), xyz(tj))), xyz(tk));
     }
-#ifndef E2_ROW_UNROLL
-#define E2_ROW_UNROLL 1          // the two output rows one after the other: one pair's state live at a time (A/B in profiles/r02_post_variants.txt)
-#endif
-    constexpr int kRowUnroll = E2_ROW_UNROLL;
-#pragma unroll kRowUnroll
+    // the two output rows one after the other: one pair's state live at a time (A/B in profiles/r02_post_variants.txt)
+#pragma unroll 1
     for (int row = 0; row < 2; ++row) {                              // output rows oy (pp.y = .25) and oy+1 (pp.y = .75)
         const float ppy = row ? 0.75f : 0.25f;
         const int y = oy + row;

@@ -34,9 +34,7 @@ __device__ __forceinline__ vqshadow::Px4 px4(float4 v) { vqshadow::Px4 r; r.x = 
 // One thread per pixel; rows strided over the grid. 32 B/pixel in (position, normal), 8 B/pixel out; the shadow maps are
 // L2-resident side data. Bound by instruction issue: ~45 instructions per cube tap (face selection, two correctly rounded
 // quotients, texel address, depth comparison), ~10 per 2-D tap.
-#ifndef PCF_MIN_BLOCKS
-#define PCF_MIN_BLOCKS 8
-#endif
+constexpr int PCF_MIN_BLOCKS = 8;
 __global__ void __launch_bounds__(128, PCF_MIN_BLOCKS) shadow_pcf_kernel(const __grid_constant__ PcfParams P) {
     const int x = blockIdx.x * blockDim.x + threadIdx.x;
     const int cx = min(x, P.width - 1);          // whole warps stay alive (pcf_record votes across the warp): a lane past the row's end

@@ -132,9 +132,7 @@ __device__ __forceinline__ int wrap_index(int i, int n) {           // general m
     return r < 0 ? r + n : r;
 }
 
-#ifndef SURF_MIN_BLOCKS
-#define SURF_MIN_BLOCKS 4
-#endif
+constexpr int SURF_MIN_BLOCKS = 4;
 struct TexR { const uint32_t* p; int w, h, levels; };               // a descriptor in registers
 __device__ __forceinline__ TexR load_tex(const DevTex* d) {
     const uint4 v = __ldg((const uint4*)d);
@@ -230,14 +228,6 @@ __device__ __forceinline__ uint64_t l2_policy_evict_last() {
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
     uint64_t p; asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p)); return p;
 }
-#ifndef SURF_L2_HINTS
-#define SURF_L2_HINTS 1
-#endif
-#if !SURF_L2_HINTS
-__device__ __forceinline__ uint32_t ld_texel(const uint32_t* p, uint64_t) { return __ldg(p); }
-__device__ __forceinline__ float4 ld_once(const float4* p, uint64_t) { return ld_stream(p); }
-__device__ __forceinline__ void st_once(float4* p, float4 v, uint64_t) { st_stream(p, v); }
-#else
 __device__ __forceinline__ uint32_t ld_texel(const uint32_t* p, uint64_t pol) {
     uint32_t r; asm volatile("ld.global.nc.L2::cache_hint.b32 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(pol)); return r;
 }
@@ -251,7 +241,6 @@ __device__ __forceinline__ void st_once(float4* p, float4 v, uint64_t pol) {
     asm volatile("st.global.L1::no_allocate.L2::cache_hint.v4.f32 [%0], {%1,%2,%3,%4}, %5;"
                  :: "l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "l"(pol) : "memory");
 }
-#endif
 
 // ---- record path: every map of the material in one 16-byte texel record ---------------------------------------------------
 // byte C of a texel word as the float 2^23 + byte (PRMT only); differences of two such values are the exact byte differences,
@@ -495,14 +484,8 @@ __device__ __forceinline__ void shade_surface_pixel(const SurfArgs& A, int x, in
 // material pixels for a second pass inside the block (0.49 ms) or for a second small launch (0.45 ms) against 0.37 ms in place —
 // the majority paths dominate the instruction count, not the stray lanes; and a persistent kernel with the interpolant planes on a
 // TMA / mbarrier ring like K1's (0.49 ms) — the waits are on the texel and SSAO loads, not on the interpolants, and 92 KB of code
-// with every warp of an SM somewhere else in it stalls on instruction fetch.
-// SURF_TILES > 1: consecutive 32x8 tiles (stacked in y) per block, the interpolants and the SSAO texel of the NEXT tile requested
-// before the current tile is shaded, so that their HBM latency (43 % of the kernel's long-scoreboard stalls) runs under a tile of
-// sampling and filtering. Measured and NOT the default: 13 more live registers cost more in spills than the overlap returns
-// (2 tiles: 0.412 ms at 64 registers, 0.397 at 80; 4 tiles: 0.401; 1 tile: 0.383).
-#ifndef SURF_TILES
-#define SURF_TILES 1
-#endif
+// with every warp of an SM somewhere else in it stalls on instruction fetch. Several tiles per block, each prefetching the
+// next tile's interpolants, were slower too: the extra live registers spill (profiles/r02_surface_variants.txt).
 struct SurfTexels { float4 pu, nv, tm; float ssao; };
 __device__ __forceinline__ SurfTexels surface_fetch(const SurfArgs& A, int x, int y, uint64_t once) {
     const int W = A.posU.w, H = A.posU.h;
@@ -526,26 +509,20 @@ __device__ __forceinline__ SurfTexels surface_fetch(const SurfArgs& A, int x, in
 __global__ void __launch_bounds__(256, SURF_MIN_BLOCKS) surface_kernel(const __grid_constant__ SurfArgs A) {
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int x = blockIdx.x * 32 + (warp & 1) * 16 + (lane & 15);
-    const int yBase = A.tileY0 + blockIdx.y * (8 * SURF_TILES) + (warp >> 1) * 2 + (lane >> 4);
+    const int y = A.tileY0 + blockIdx.y * 8 + (warp >> 1) * 2 + (lane >> 4);
     const int W = A.posU.w, H = A.posU.h;
     const uint64_t once = l2_policy_evict_first();
-    SurfTexels nxt = surface_fetch(A, x, yBase, once);
-#pragma unroll 1
-    for (int it = 0; it < SURF_TILES; ++it) {
-        const int y = yBase + 8 * it;
-        const SurfTexels cur = nxt;
-        if (it + 1 < SURF_TILES && y + 8 - (lane >> 4) - (warp >> 1) * 2 < A.rowEnd) nxt = surface_fetch(A, x, y + 8, once);   // block-uniform test
-        const float ru = cur.pu.w, rv = cur.nv.w;
-        // fine quad derivatives of the RAW uv: horizontal partner = lane^1, vertical = lane^16
-        const float ruX = __shfl_xor_sync(0xffffffffu, ru, 1), rvX = __shfl_xor_sync(0xffffffffu, rv, 1);
-        const float ruY = __shfl_xor_sync(0xffffffffu, ru, 16), rvY = __shfl_xor_sync(0xffffffffu, rv, 16);
-        const float sx = (lane & 1) ? -1.0f : 1.0f, sy = (lane & 16) ? -1.0f : 1.0f;   // (odd - even) regardless of which I am
-        const float dRawUdx = (ruX - ru) * sx, dRawVdx = (rvX - rv) * sx;
-        const float dRawUdy = (ruY - ru) * sy, dRawVdy = (rvY - rv) * sy;
-        if (x < W && y < H && y >= A.rowBegin && y < A.rowEnd) {
-            const int mi = min(max((int)cur.tm.w, 0), A.nMats - 1);
-            shade_surface_pixel(A, x, y, mi, cur.pu, cur.nv, cur.tm, cur.ssao, dRawUdx, dRawVdx, dRawUdy, dRawVdy, once);
-        }
+    const SurfTexels cur = surface_fetch(A, x, y, once);
+    const float ru = cur.pu.w, rv = cur.nv.w;
+    // fine quad derivatives of the RAW uv: horizontal partner = lane^1, vertical = lane^16
+    const float ruX = __shfl_xor_sync(0xffffffffu, ru, 1), rvX = __shfl_xor_sync(0xffffffffu, rv, 1);
+    const float ruY = __shfl_xor_sync(0xffffffffu, ru, 16), rvY = __shfl_xor_sync(0xffffffffu, rv, 16);
+    const float sx = (lane & 1) ? -1.0f : 1.0f, sy = (lane & 16) ? -1.0f : 1.0f;   // (odd - even) regardless of which I am
+    const float dRawUdx = (ruX - ru) * sx, dRawVdx = (rvX - rv) * sx;
+    const float dRawUdy = (ruY - ru) * sy, dRawVdy = (rvY - rv) * sy;
+    if (x < W && y < H && y >= A.rowBegin && y < A.rowEnd) {
+        const int mi = min(max((int)cur.tm.w, 0), A.nMats - 1);
+        shade_surface_pixel(A, x, y, mi, cur.pu, cur.nv, cur.tm, cur.ssao, dRawUdx, dRawVdx, dRawUdy, dRawVdy, once);
     }
 }
 
@@ -710,7 +687,7 @@ extern "C" int vq_gbuffer_from_materials(VqContext* ctx, const VqSurfaceInputs* 
     A.mats = table->dev; A.nMats = table->count;
     A.ambient = ambient_factor; A.alphaMask = alpha_mask;
     A.rowBegin = row_begin; A.rowEnd = row_end; A.tileY0 = row_begin & ~1;
-    const dim3 grid((W + 31) / 32, (row_end - A.tileY0 + 8 * SURF_TILES - 1) / (8 * SURF_TILES));
+    const dim3 grid((W + 31) / 32, (row_end - A.tileY0 + 7) / 8);
     surface_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(A);
     return vq_check_launch("gbuffer_from_materials");
 }
